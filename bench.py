@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200-native Enoki backend.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (N=1 and every rank of N>1, weak scaling): BASELINE.json configs[1] =
 "CUDAArray<float> 64M-elem fused arith+exp/sin chain, cuda_eval()":
@@ -44,6 +44,7 @@ N_ELEMS = 1 << 26
 C2_NODES = 9            # fma, mul, neg, exp, fma, sin, abs, sqrt, fma (what the runtime counts as ops=)
 C2_BYTES_PER_ELEM = 20  # 4 input streams + 1 output stream, fp32 (SURVEY 8d)
 C4 = dict(levels=80, per_level=128, width=131072)
+DUMP_ELEMS = 1 << 22    # --dump-outputs: at most 16 MiB of float32 output
 
 
 def P(a):
@@ -291,7 +292,17 @@ def main():
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-e2e", action="store_true", help="profiling aid: leave out the host-buffer leg")
     ap.add_argument("--skip-extras", action="store_true", help="profiling aid: leave out C3 / small / C5 / C1 objects")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy: out.npy (float32; the "
+                         f"whole output up to {DUMP_ELEMS} elements, beyond that the elements at a fixed seeded sample of "
+                         "indices) and hsum.npy (the loss scalar, all-reduced when N>1); rank 0 only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path")
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
 
     if args.impl == "reference":
@@ -397,6 +408,9 @@ def main():
     ms_per_step = ms / args.steps
     value = world * n * C2_NODES / (ms_per_step * 1e-3) / 1e6
     loss_val = float(keep[1].numpy()[0])
+    dump = None
+    if args.dump_outputs and rank == 0:
+        dump = {"out": sample_output(keep[0].numpy()), "hsum": keep[1].numpy().astype(np.float32)}
     del keep
 
     # ---- roofline of the dominant kernel: per-launch CUDA events on the launch stream
@@ -570,8 +584,8 @@ def main():
       try:
         c, quota = best_cpu_config(N_ELEMS)
         r = cpu_wall_rate(c, 16)
-        c1 = CpuC2(1 << 24, 1); c1.run(1)
-        r1 = cpu_wall_rate(c1, 2)
+        single = CpuC2(1 << 24, 1); single.run(1)
+        r1 = cpu_wall_rate(single, 2)
         cpu = {"value": r * C2_NODES / 1e6, "unit": "M array-ops/s", "cores": c.threads, "kind": c.kind,
                "sample": f"16 passes over all 2^26 elements split over {c.threads} threads (host exposes {os.cpu_count()} CPUs, CPU quota "
                          f"{quota}; DRAM resident; reference vectorize() form, AVX2+FMA -ffp-contract=fast; wall clock); "
@@ -594,16 +608,29 @@ def main():
             "backward": backward, "backward_width_16384": backward_narrow, "histogram": hist, "c5": c5, "c1_cpu": c1, "small": small, "wall_ms_per_step": wall_ms / args.steps, "loss_checksum": loss_val,
         }
         print(json.dumps(line), flush=True)
+    if dump is not None:
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
     if dist is not None:
         dist.barrier()
         dist.destroy_process_group()
 
 
+def sample_output(a):
+    """`a` itself when it has at most DUMP_ELEMS elements, else its elements at DUMP_ELEMS-or-fewer fixed indices (seeded,
+    ascending, depending only on len(a)), so that two builds run with the same arguments dump comparable files."""
+    if len(a) <= DUMP_ELEMS:
+        return a
+    idx = np.unique(np.random.default_rng(0).integers(0, len(a), DUMP_ELEMS))
+    return a[idx]
+
+
 def _qualification_timing():
     """What enoki_b200/ek_qualify measured when ek_init() qualified the fast kernel on this machine (general vs fast kernel,
     C2 and C3 at 2^24 elements, device time of the sweep launch); None when the qualification was skipped or failed earlier."""
-    try:
-        return json.load(open(os.path.join(ROOT, "enoki_b200", ".ek_fast_timing.json")))
+    try:     # written by ek_init() (csrc/ek_runtime.cpp) into the temporary directory
+        tmp = os.environ.get("TMPDIR") or "/tmp"
+        return json.load(open(os.path.join(tmp, f"ek_b200_fast_timing_{os.getuid()}.json")))
     except Exception:
         return None
 

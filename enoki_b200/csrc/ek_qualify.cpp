@@ -374,7 +374,7 @@ int main(int argc, char **argv) {
     if (bad) return 1;
     /* correct -- but is it faster here?  The fast kernel exists to beat the general one; if it does not on this GPU (C2, the
        headline workload, 2^24 elements, device time of the sweep launch), the general kernel stays in charge.  The numbers
-       go into a small file next to the library so that bench.py can report them. */
+       go into the small file named by argv[1] (ek_runtime.cpp: in the temporary directory) so that bench.py can report them. */
     double g2 = 0, g3 = 0, f2 = 0, f3 = 0;
     const size_t nt = (size_t) 1 << 24;
     ek_set_fast_mode(0); time_c2_c3(nt, g2, g3);

@@ -87,7 +87,9 @@ int ek_set_device(int ordinal) {
    test-suite, and through the fast kernel -- and compares the results bit for bit.  Only when every comparison agrees
    (exit status 0, within 150 s) is the fast kernel used; a wrong result, a CUDA error, a watchdog trap or a crash of the
    child all leave this process on the general kernels, with one line on stderr.  The verdict is remembered in a stamp
-   file keyed on the library file and the GPU name, so the battery runs once per machine, not once per process.
+   file keyed on the library file and the GPU name, so the battery runs once per machine, not once per process.  The
+   stamp and the helper's timings go to $TMPDIR (or /tmp), never next to the library: the installed tree may be
+   read-only, and using it must not change it.
    EK_FAST=0 / EK_FAST=1 skip the qualification and force the answer (the child itself runs with EK_FAST=0 and switches
    modes through ek_set_fast_mode()). */
 static std::string lib_path() {
@@ -109,10 +111,11 @@ static int decide_fast_mode(const char *gpu_name) {
     }
     char key[512];
     snprintf(key, sizeof(key), "lib %lld %lld gpu %s", (long long) st_lib.st_size, (long long) st_lib.st_mtime, gpu_name);
-    std::string stamps[2] = { dir + "/.ek_fast_qualified", "/tmp/ek_b200_fast_qualified_" + std::to_string((long) getuid()) };
-    for (const std::string &sp : stamps) {
-        FILE *f = fopen(sp.c_str(), "r");
-        if (!f) continue;
+    const char *tmpdir = getenv("TMPDIR");
+    const std::string state = std::string(tmpdir && *tmpdir ? tmpdir : "/tmp") + "/ek_b200_fast_";
+    const std::string uid = std::to_string((long) getuid());
+    const std::string stamp = state + "qualified_" + uid;
+    if (FILE *f = fopen(stamp.c_str(), "r")) {
         char line[600] = { 0 }; int verdict = -1;
         if (fgets(line, sizeof(line), f)) { size_t l = strlen(line); while (l && (line[l - 1] == '\n' || line[l - 1] == '\r')) line[--l] = 0; }
         if (fscanf(f, "%d", &verdict) != 1) verdict = -1;
@@ -121,7 +124,8 @@ static int decide_fast_mode(const char *gpu_name) {
     }
     /* run the battery in a child process (this process may already hold CUDA state: no fork-without-exec) */
     pid_t pid = 0;
-    const std::string timing_file = dir + "/.ek_fast_timing.json";
+    const std::string timing_file = state + "timing_" + uid + ".json";     /* read by bench.py */
+    unlink(timing_file.c_str());          /* a failed battery writes none: never leave another library's timings there */
     char *argv[] = { const_cast<char *>(helper.c_str()), const_cast<char *>(timing_file.c_str()), nullptr };
     std::vector<std::string> envs;
     for (char **e = environ; e && *e; ++e) if (strncmp(*e, "EK_FAST=", 8) != 0) envs.push_back(*e);
@@ -147,14 +151,11 @@ static int decide_fast_mode(const char *gpu_name) {
                     !done ? "timeout" : WIFSIGNALED(status) ? "child crashed" :
                     (WIFEXITED(status) && WEXITSTATUS(status) == 4) ? "correct, but not faster than the general kernel here" : "results differ / CUDA error, see above");
     }
-    for (const std::string &sp : stamps) {
-        const std::string tmp = sp + "." + std::to_string((long) getpid());
-        FILE *f = fopen(tmp.c_str(), "w");
-        if (!f) continue;
+    const std::string tmp = stamp + "." + std::to_string((long) getpid());
+    if (FILE *f = fopen(tmp.c_str(), "w")) {
         fprintf(f, "%s\n%d\n", key, verdict);
         fclose(f);
-        if (rename(tmp.c_str(), sp.c_str()) == 0) break;
-        unlink(tmp.c_str());
+        if (rename(tmp.c_str(), stamp.c_str()) != 0) unlink(tmp.c_str());
     }
     return verdict;
 }

@@ -4,17 +4,27 @@
 the .npz files are committed.
 
     python tests/golden/make_golden.py
+
+The tests import make_tape() and ref_math_inputs() from here to regenerate inputs, so the reference
+library is only loaded when vectors are written.
 """
 import ctypes
+import hashlib
 import os
+import subprocess
 
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-R = ctypes.CDLL(os.path.join(ROOT, "oracle", "_ref", "libenoki_ref.so"))
+R = None
 P = lambda a: a.ctypes.data_as(ctypes.c_void_p)
 SZ = ctypes.c_size_t
+
+
+def load_ref():
+    global R
+    R = ctypes.CDLL(os.path.join(ROOT, "oracle", "_ref", "libenoki_ref.so"))
 
 
 def unary(name, x):
@@ -24,6 +34,7 @@ def unary(name, x):
 
 
 def main():
+    load_ref()
     rng = np.random.default_rng(20260922)
     # --- C2: fused chain (SURVEY 8d) on 4099 elements
     n = 4099
@@ -93,7 +104,70 @@ def main():
         assert R.ref_ad_expr(which, P(x), SZ(len(x)), P(v), P(gr)) == 0
         d[f"val{which}"] = v; d[f"grad{which}"] = gr
     np.savez_compressed(os.path.join(HERE, "ad_expr.npz"), **d)
+    ref_compare()
     print("golden vectors written to", HERE)
+
+
+MATH_SAMPLE = 2048
+
+
+def ref_math_inputs():
+    """[(name, oracle selector, float32 arguments)]: 2^18 arguments per function, special values first."""
+    rng = np.random.default_rng(1)
+    n = 1 << 18
+    cases = []
+    for name, which, gen in [("sin", 0, lambda: rng.uniform(-8192, 8192, n)), ("cos", 1, lambda: rng.uniform(-8192, 8192, n)),
+                             ("exp", 2, lambda: rng.uniform(-100, 100, n)), ("log", 3, lambda: np.exp(rng.uniform(-80, 80, n))),
+                             ("sqrt", 4, lambda: rng.uniform(0, 1e10, n))]:
+        x = gen().astype(np.float32)
+        x[:8] = [0, -0.0, np.inf, -np.inf, np.nan, 1, -1, 1e-40]
+        cases.append((name, which, x))
+    return cases
+
+
+def ref_math_sample(n):
+    """Indices of the stored sample: the special values and a seeded draw from the rest."""
+    return np.unique(np.concatenate([np.arange(8), np.random.default_rng(2).integers(8, n, MATH_SAMPLE - 8)]))
+
+
+def digest_f32(a):
+    """SHA-256 of a float32 array with every NaN written as the one quiet NaN (NaN == NaN in the comparisons)."""
+    a = np.array(a, np.float32)
+    a[np.isnan(a)] = np.nan
+    return hashlib.sha256(a.tobytes()).hexdigest()
+
+
+def ref_compare():
+    """What the oracle is compared with: the reference's float32 math on ref_math_inputs() (a sample of arguments and
+    results, and the SHA-256 of every result), its rcp / rsqrt at a sample of the GPU test's arguments, the reference
+    tape's gradients on make_tape(rng 5, 7, 12, 333), and the
+    planner listings that tests/cpp/shim_plan (C++ code through include/enoki/cuda.h under the reference headers) prints."""
+    d = {}
+    for name, _, x in ref_math_inputs():
+        out = unary(name, x)
+        idx = ref_math_sample(len(x))
+        d["idx"] = idx.astype(np.uint32)
+        d[f"{name}_x"] = x[idx]; d[f"{name}_ref"] = out[idx]; d[f"{name}_sha256"] = np.array(digest_f32(out))
+    np.savez_compressed(os.path.join(HERE, "ref_math.npz"), **d)
+
+    # rcp / rsqrt of tests/test_gpu_eval.py::test_unary_f32 (rcpps / rsqrtps + one Newton step): a seeded sample
+    d = {}
+    for name, which, lo, hi in [("rcp", 5, -100, 100), ("rsqrt", 6, 1e-10, 1e10)]:
+        x = np.random.default_rng(which).uniform(lo, hi, 1 << 18).astype(np.float32)
+        idx = np.unique(np.random.default_rng(3).integers(0, len(x), 4096))
+        d[f"{name}_idx"] = idx.astype(np.uint32); d[f"{name}_x"] = x[idx]; d[f"{name}_ref"] = unary(name, x)[idx]
+    np.savez_compressed(os.path.join(HERE, "ref_rcp.npz"), **d)
+
+    w = 333
+    g = make_tape(np.random.default_rng(5), 7, 12, w)
+    grads = np.zeros(len(g["want"]) * w, np.float32)
+    assert R.ref_tape_backward(len(g["node_size"]), P(g["node_size"]), len(g["src"]), P(g["src"]), P(g["dst"]), P(g["weights"]),
+                               P(g["woff"]), P(g["wsize"]), int(g["root"]), len(g["want"]), P(g["want"]), P(grads), 1) == 0
+    np.savez_compressed(os.path.join(HERE, "ref_tape.npz"), grads=grads)
+
+    out = subprocess.run([os.path.join(ROOT, "tests", "cpp", "shim_plan")], capture_output=True, text=True, check=True).stdout
+    with open(os.path.join(HERE, "shim_plan.txt"), "w") as f:
+        f.write(out)
 
 
 def make_tape(rng, L, K, w, zero_frac=0.01):
